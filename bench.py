@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                 # configs[1]: this repo's CUDA path (headline)
     python bench.py --impl reference --gpus N --steps K ...        # the same workload on the CPU oracle (host cores)
     python bench.py --config c3|c4|c5|4k|rich ...                  # the other shapes, each with its own roofline
+    python bench.py ... --dump-outputs DIR                         # + what the last timed step computed, as DIR/*.npy
 
 Workloads (no real doom1.wad / doom2.wad exists in the environment: synthetic stand-ins of the same scale; set
 B2D_IWAD=/path/doom1.wad to run c2 on a real one):
@@ -15,9 +16,13 @@ B2D_IWAD=/path/doom1.wad to run c2 on a real one):
                    overlapped with rendering (b2d_render_sharded); render-only / gather-only / joint reported separately
   4k   c2 at 3840x2160 (100-pose batches);   rich: c2 on the content-rich generated level (masked middles, sprites,
                    animated / scrolling / flashing content)
-One "step" is one pass of the hot path over the configuration's pose set.  `value` is device-resident throughput (poses
-already in HBM, frames written to HBM); `e2e` (c2) goes through b2d_render with pinned HOST buffers -- host poses in,
-host frames out, both copies inside the timed region.
+One "step" is one pass of the hot path over the configuration's pose set; --steps sets how many are timed.  `value` is
+device-resident throughput (poses already in HBM, frames written to HBM); `e2e` (c2) goes through b2d_render with
+pinned HOST buffers -- host poses in, host frames out, both copies inside the timed region.
+
+--dump-outputs DIR writes, after the timed steps, what the last step handed its caller (the index frames, the RGBA
+frames with --rgba, c5's per-frame checksums) as float32 / float64 .npy files: a fixed, seeded sample of at most 64 MB.
+Poses and levels are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -28,6 +33,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -113,6 +119,48 @@ def ncu_traffic():
             return json.load(f).get("raster_dram_bytes_per_launch")
     except Exception:  # noqa: BLE001
         return None
+
+
+DUMP_MAX_BYTES = 64 * 1000 * 1000
+DUMP_SEED = 2024
+
+
+def dump_share(n_outputs):
+    """Bytes each of `n_outputs` outputs may take in DIR (the .npy headers fit in what is held back)."""
+    return (DUMP_MAX_BYTES - (64 << 10)) // n_outputs
+
+
+def sample_output(name, t, share, dtype=np.float32):
+    """What --dump-outputs keeps of the output `t` (a torch tensor whose first axis is the frame) in at most `share` bytes
+    of `dtype`: the whole output when it fits, else a fixed, seeded sample of it -- `<name>_values`, values at random
+    positions over the whole output, so that every frame is represented, and `<name>_frames`, whole frames at random
+    positions, as many as the rest of the share holds."""
+    import torch
+
+    def host(x):
+        return x.cpu().numpy().astype(dtype)
+
+    size = np.dtype(dtype).itemsize
+    if t.numel() * size <= share:
+        return {name: host(t)}
+    rng = np.random.default_rng([DUMP_SEED, zlib.crc32(name.encode())])
+    n, total = t.shape[0], t.numel()
+    nval = min(total, share // size // 8)
+    k = min(n, (share - nval * size) // (total // n * size))
+    if k == 0:
+        nval = share // size
+    pos = torch.from_numpy(np.sort(rng.integers(0, total, nval))).to(t.device)
+    out = {name + "_values": host(t.reshape(-1)[pos])}
+    if k:
+        out[name + "_frames"] = host(t[torch.from_numpy(np.sort(rng.choice(n, k, replace=False))).to(t.device)])
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -303,7 +351,7 @@ def roofline_of(raster_ms_per_launch_set, alg_bytes, walk_ms, note, kernel="b2d_
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b2d", choices=["b2d", "reference"])
     ap.add_argument("--config", default="c2", choices=["c2", "c3", "c4", "c5", "4k", "rich"])
@@ -324,7 +372,13 @@ def main():
                          "first CTAs of batch k+1 fill the SMs that the last CTAs of batch k leave idle (1 = one stream, one buffer)")
     ap.add_argument("--rgba", action="store_true", help="c2: also materialise RGBA8 frames in HBM (5 B/pixel; not the headline config)")
     ap.add_argument("--gather-frames", type=int, default=0, help="c2, N>1: frames per rank in a separate all-gather timing (0 = off; see --config c5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (rank 0's "
+                    "outputs) as DIR/<name>.npy: float32 (float64 for c5's checksums), a fixed, seeded sample of at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b2d)")
     args.warmup = max(args.warmup, 0)
     cfg = args.config
     # stdout carries the one JSON line: NCCL's version banner / debug output (NCCL_DEBUG may be set by the box) goes to stderr
@@ -383,17 +437,20 @@ def main():
         sampler = ClockSampler(local_rank)
         if rank == 0:
             sampler.start()
-        results = {}
+        results, checksums = {}, {}
         for tname in [t for t in args.transports.split(",") if t]:
             for k in ("B2D_NCCL_NO_WINDOW", "B2D_NCCL_NO_REGISTER", "B2D_GATHER"):
                 os.environ.pop(k, None)
             os.environ.update(env_of[tname])
             comm = jobs.make_comm(local_rank) if world > 1 else jobs.single_comm(local_rank)
-            r1 = jobs.run_c5(scene, poses, width, height, local_rank, comm, chunk=args.chunk, reps=max(1, min(args.steps, 3)))
+            r1 = jobs.run_c5(scene, poses, width, height, local_rank, comm, chunk=args.chunk, reps=args.steps)
             v1 = verify_c5(b2d, jobs, r1, scene, poses, width, height, rank, world)
             if not v1["all_ranks_identical"] or v1["oracle_mismatches"] or r1["status_bits"]:
                 raise SystemExit("c5 validation failed (%s): %r status %d" % (tname, v1, r1["status_bits"]))
-            r1.pop("table"); r1.pop("renderer")
+            table = r1.pop("table")
+            r1.pop("renderer")
+            if args.dump_outputs and rank == 0:
+                checksums[tname] = table.host()
             results[tname] = (r1, v1)
             comm.close()
             torch.cuda.empty_cache()
@@ -404,9 +461,12 @@ def main():
                 "render_only_fps", "gather_only_fps", "joint_fps", "joint_checked_fps", "gather_gbs_received_per_rank",
                 "joint_gbs_received_per_rank", "registration", "nccl_version")
         if rank == 0:
+            if args.dump_outputs:       # per-frame checksums of every gathered frame, [rank, frame of the rank's slice]
+                write_outputs(args.dump_outputs, sample_output("checksums", torch.from_numpy(checksums[best].astype(np.int64)),
+                                                               dump_share(1), np.float64))
             nvl = 900.0
             print(json.dumps({
-                "metric": METRIC, "value": res["joint_fps"], "unit": UNIT, "n_gpus": world, "steps": 1, "warmup": 1,
+                "metric": METRIC, "value": res["joint_fps"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": 1,
                 "ms_per_step": res["joint_ms"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                 "dtype": "u8", "data": "synthetic",
                 "config": bench_config(desc, res["per_rank"], world, scene.info,
@@ -441,7 +501,9 @@ def main():
             scenes.append(sc)
             ps = make_poses(sc, kind, n, pseed)
             poses.append(np.roll(ps, -(rank * n // max(world, 1))) if cfg != "c4" else ps)
-        steps = max(1, args.steps if cfg != "c4" else min(args.steps, 5))
+        steps = args.steps
+        dump = args.dump_outputs and rank == 0
+        dumped = {}
         sampler = ClockSampler(local_rank)
         if rank == 0:
             sampler.start()
@@ -450,9 +512,11 @@ def main():
             # one map at a time (frames of a 4K map: 8.3 GB per 1000): keep one output buffer alive
             tot = {"ms_per_pass": 0.0, "raster_ms_per_pass": 0.0, "walk_ms_per_pass": 0.0, "frames_per_pass": 0, "launches": 0, "status_bits": 0}
             bad = 0
-            for sc, ps in zip(scenes, poses):
+            for m, sc, ps in zip(mine, scenes, poses):
                 r1 = jobs.run_maps([sc], [ps], width, height, local_rank, batch, steps, args.warmup, False, args.raster_streams)
                 bad += verify_maps(r1, [sc], [ps], width, height)
+                if dump:
+                    dumped.update(sample_output(maps[m][0] + "_index", r1["outs"][0], dump_share(len(scenes))))
                 for k in tot:
                     tot[k] += r1[k]
                 del r1
@@ -461,6 +525,11 @@ def main():
         else:
             res = jobs.run_maps(scenes, poses, width, height, local_rank, batch, steps, args.warmup, cfg == "c3", args.raster_streams)
             bad = verify_maps(res, scenes, poses, width, height)
+            if dump:
+                for m, out in zip(mine, res["outs"]):
+                    dumped.update(sample_output(maps[m][0] + "_index", out, dump_share(len(scenes))))
+        if dump:
+            write_outputs(args.dump_outputs, dumped)
         clocks = sampler.stop() if rank == 0 else None
         if bad or res["status_bits"]:
             raise SystemExit("parity check failed: %d probe frame(s) differ from the oracle, status %d" % (bad, res["status_bits"]))
@@ -570,6 +639,15 @@ def main():
     join()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:        # the buffers the last step rastered into, before anything else writes them
+        b = (turn[0] - 1) % nbuf if pipelined else 0
+        outs = {"index": d_index_all[b]}
+        if args.rgba:                          # RGBA8 per pixel, as channels
+            outs["rgba"] = d_rgba_all[b].view(torch.uint8).reshape(n, height, width, 4)
+        dumped = {}
+        for name, t in outs.items():
+            dumped.update(sample_output(name, t, dump_share(len(outs))))
+        write_outputs(args.dump_outputs, dumped)
     if pipelined:                              # the walk issued by the last step belongs to a step that never comes
         r.raster_device(pending[0], d_index.data_ptr(), d_rgba.data_ptr() if args.rgba else 0, stream)
         torch.cuda.synchronize()

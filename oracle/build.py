@@ -12,6 +12,7 @@ import hashlib
 import os
 import subprocess
 import sys
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "b2d_oracle.c")
@@ -49,6 +50,11 @@ def needs_build() -> bool:
 def build(force: bool = False) -> str:
     if not force and not needs_build():
         return OUT
+    if not os.access(HERE, os.W_OK):
+        # a read-only tree whose library was built for another host: this host's build goes to a temporary directory
+        out = os.path.join(tempfile.mkdtemp(prefix="b2d_oracle_"), os.path.basename(OUT))
+        subprocess.check_call(["gcc"] + FLAGS + ["-o", out, SRC])
+        return out
     subprocess.check_call(["gcc"] + FLAGS + ["-o", OUT, SRC])
     with open(HOST, "w") as f:
         f.write(host_signature() + "\n")
