@@ -226,6 +226,22 @@ static void draw_sky(Frame *f, int x, int ya, int yb) {
     }
 }
 
+/* floor(n * invF / 2^40), exact: n * invF itself exceeds 64 bits on low, wide views (W/F > ~31), so the product is
+ * taken in two halves, n = hi * 2^20 + lo with 0 <= lo < 2^20 */
+static inline int32_t mul_invF_q40(int64_t n, uint32_t invF) {
+    const int64_t hi = asr64(n, 20), lo = n - hi * ((int64_t)1 << 20);
+    return (int32_t)asr64(hi * (int64_t)invF + asr64(lo * (int64_t)invF, 20), 20);
+}
+
+/* direction of column x's ray, Q18 (DESIGN.md C8): (cos*F + sin*c2)/F, (sin*F - cos*c2)/F with c2 = 2x+1-W */
+static inline void plane_dir(int32_t cosq, int32_t sinq, const b2o_view *vw, uint32_t invF, int x, int32_t *ax, int32_t *ay) {
+    const int64_t c2 = 2 * (int64_t)x + 1 - vw->W;
+    const int64_t nx = asr64((int64_t)cosq * vw->F + (int64_t)sinq * c2, 4);
+    const int64_t ny = asr64((int64_t)sinq * vw->F - (int64_t)cosq * c2, 4);
+    *ax = mul_invF_q40(nx, invF);
+    *ay = mul_invF_q40(ny, invF);
+}
+
 static void draw_plane(Frame *f, int x, int ya, int yb, int32_t h, int32_t flat, int lightb) {
     const Scene *sc = f->sc;
     if (ya >= yb) return;
@@ -233,16 +249,12 @@ static void draw_plane(Frame *f, int x, int ya, int yb, int32_t h, int32_t flat,
     flat = flat_now(f, flat);
     if (flat < 0 || flat >= sc->nflats) return;               /* missing flat: pixels stay void */
     const uint8_t *px = sc->flats + 4096 * (size_t)flat;
-    int W = f->vw.W;
     int64_t hrel = clamp64(((int64_t)h << 16) - f->pose.z, -((int64_t)1 << 27), (int64_t)1 << 27);
     uint64_t a = (uint64_t)(hrel < 0 ? -hrel : hrel);
     const int64_t key = (((int64_t)h << 9) | (int64_t)(lightb & 0x1FF)) + 1;
-    /* direction of this column's ray, Q18 (DESIGN.md C8): (cos*F + sin*c2)/F, (sin*F - cos*c2)/F with c2 = 2x+1-W */
-    const int64_t c2 = 2 * (int64_t)x + 1 - W;
-    const int64_t nx = asr64((int64_t)f->cosq * f->vw.F + (int64_t)f->sinq * c2, 4);
-    const int64_t ny = asr64((int64_t)f->sinq * f->vw.F - (int64_t)f->cosq * c2, 4);
-    const uint32_t ax = (uint32_t)(int32_t)asr64(nx * (int64_t)f->invF, 40);
-    const uint32_t ay = (uint32_t)(int32_t)asr64(ny * (int64_t)f->invF, 40);
+    int32_t dx, dy;
+    plane_dir(f->cosq, f->sinq, &f->vw, f->invF, x, &dx, &dy);
+    const uint32_t ax = (uint32_t)dx, ay = (uint32_t)dy;
     const uint32_t bu = (uint32_t)f->pose.x << 10, bv = (uint32_t)f->pose.y << 10;
     for (int y = ya; y < yb; y++) {
         uint32_t *pr = f->prow + 2 * (size_t)y;
@@ -569,6 +581,13 @@ void b2o_view_init(b2o_view *v, int W, int H, double tan_half_fovy) {
     v->W = W; v->H = H;
     v->FY2 = (int32_t)(fy2 + 0.5);
     v->F = (int32_t)(fx2 + 0.5);
+}
+
+/* direction of every column's ray at yaw `angle`, Q18, as draw_plane uses it (DESIGN.md C8): out[2x] = ax, out[2x+1] = ay */
+void b2o_plane_dirs(const b2o_view *vw, uint32_t angle, int32_t *out) {
+    int32_t c, s;
+    b2o_sincos_q30(angle, &c, &s);
+    for (int x = 0; x < vw->W; x++) plane_dir(c, s, vw, (uint32_t)(4294967296ULL / (uint64_t)vw->F), x, &out[2 * x], &out[2 * x + 1]);
 }
 
 /* light_ov: NULL, or one int16 per sector (oracle/scene.py sector_lights_at(blob, tics)) */

@@ -33,6 +33,7 @@ def lib():
         L.b2o_crc32.argtypes = [ctypes.c_void_p, ctypes.c_size_t]
         L.b2o_crc32.restype = ctypes.c_uint32
         L.b2o_sincos_q30.argtypes = [ctypes.c_uint32, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]
+        L.b2o_plane_dirs.argtypes = [ctypes.POINTER(View), ctypes.c_uint32, ctypes.c_void_p]
         _lib = L
     return _lib
 
@@ -91,3 +92,11 @@ def sincos_q30(angle: int) -> Tuple[int, int]:
     c, s = ctypes.c_int32(), ctypes.c_int32()
     lib().b2o_sincos_q30(angle & 0xFFFFFFFF, ctypes.byref(c), ctypes.byref(s))
     return c.value, s.value
+
+
+def plane_dirs(view: View, angle: int) -> np.ndarray:
+    """(W, 2) int32: direction (ax, ay) of every screen column's ray at yaw `angle` (BAM), Q18, as the flat texel rule
+    uses it (DESIGN.md C8)."""
+    out = np.zeros((view.W, 2), dtype=np.int32)
+    lib().b2o_plane_dirs(ctypes.byref(view), angle & 0xFFFFFFFF, out.ctypes.data)
+    return out

@@ -261,14 +261,22 @@ B2D_HD int32_t wall_hrel(int32_t h, int32_t pose_z) {
 // (unit forward component).  Per column (once per frame): dir in Q18.  Per row and plane: z in Q8 and the light row.
 // Per pixel: U = (pose.x << 10) + z * dirx, V likewise -- two 32-bit multiply-adds, Q26 modulo 64 texels by wrap-around.
 struct PlaneDir { int32_t ax, ay; };                     // Q18
+// floor(n * invF / 2^40) without a 128-bit product: n * invF reaches 2^58 * (1 + |c2|/F) and overflows 64 bits once
+// W/F > ~31 (low, wide views), so n is split as hi * 2^20 + lo, 0 <= lo < 2^20, and
+// floor((hi*invF*2^20 + lo*invF) / 2^40) = (hi*invF + ((lo*invF) >> 20)) >> 20.  |hi*invF| < 2^38 * (1 + W/F) < 2^50
+// for every F >= 2; the result is at most 2^18 * (1 + W/F) < 2^30 in magnitude.
+B2D_HD int32_t mul_invF_q40(int64_t n, uint32_t invF) {
+    const int64_t hi = n >> 20, lo = n & 0xFFFFF;
+    return (int32_t)((hi * (int64_t)invF + ((lo * (int64_t)invF) >> 20)) >> 20);
+}
 B2D_HD PlaneDir plane_dir(const FrameConst &f, const View &vw, int x, uint32_t invF) {
     const int64_t c2 = 2 * (int64_t)x + 1 - vw.W;
-    // (cos*F + sin*c2) / F and (sin*F - cos*c2) / F, Q30 -> Q18 through invF = floor(2^32 / F); >> 4 first keeps 64 bits
+    // (cos*F + sin*c2) / F and (sin*F - cos*c2) / F, Q30 -> Q18 through invF = floor(2^32 / F)
     const int64_t nx = ((int64_t)f.cosq * vw.F + (int64_t)f.sinq * c2) >> 4;
     const int64_t ny = ((int64_t)f.sinq * vw.F - (int64_t)f.cosq * c2) >> 4;
     PlaneDir d;
-    d.ax = (int32_t)((nx * (int64_t)invF) >> 40);
-    d.ay = (int32_t)((ny * (int64_t)invF) >> 40);
+    d.ax = mul_invF_q40(nx, invF);
+    d.ay = mul_invF_q40(ny, invF);
     return d;
 }
 struct PlaneRow { uint32_t z8q; int32_t z8; };           // depth Q8 (for the texel), depth in 1/8 units (for the light row)

@@ -511,6 +511,18 @@ extern "C" void hostcheck_lights(const uint8_t *blob, uint32_t tics, int16_t *ou
 
 extern "C" void hostcheck_sincos(uint32_t angle, int32_t *c, int32_t *s) { sincos_q30(angle, *c, *s); }
 
+// the product's flat-texel ray direction (plane_dir, Q18) of every column, as the raster kernel computes it per column:
+// out[2x] = ax, out[2x+1] = ay
+extern "C" void hostcheck_plane_dirs(const View *vw, const Pose *pose, int32_t *out) {
+    FrameConst fc;
+    frame_setup(*pose, fc);
+    const uint32_t invF = (uint32_t)(4294967296ULL / (uint64_t)vw->F);
+    for (int x = 0; x < vw->W; x++) {
+        const PlaneDir d = plane_dir(fc, *vw, x, invF);
+        out[2 * x] = d.ax; out[2 * x + 1] = d.ay;
+    }
+}
+
 // lock-step iteration statistics for a strip width (design exploration; test-only)
 extern "C" int hostcheck_stats(const uint8_t *blob, const View *vw, const Pose *poses, int n, int strip_width,
                                long long *out4) {
